@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: Next3D generator forward (TriPlaneGenerator.synthesis) images/sec on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--batch B] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; seeded random-init weights of the FFHQ-512 architecture (172.8 M parameters), synthetic
 latents, the demo FLAME mesh, synthetic all-ones eye mask, noise_mode='const', sampler uniforms from the in-kernel RNG):
@@ -14,6 +14,8 @@ A "step" = one synthesis() call on one batch per GPU (c4: the whole clip; c5: on
 `value` = whole-job images/s with inputs resident in HBM; `e2e` = the same through the public API with pinned HOST
 inputs (H2D inside the timed region) and the final images read back to the host (D2H inside the timed region).
 The default N=1 run also reports c3 / c4 / c5 under `other_configs` (short runs; the headline stays c2).
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (see _dump_outputs); the inputs,
+weights and sampler seeds depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times the CPU oracle port (the reference itself is Python that cannot travel to the GPU box; the oracle
 is pinned bit-exactly against it, tests/test_oracle_vs_reference.py) on the host cores.
 """
@@ -78,6 +80,27 @@ def _emit(line):
     out = _JSON_OUT or sys.stdout
     out.write(json.dumps(line) + '\n')
     out.flush()
+
+
+DUMP_BYTES = 60 * 10 ** 6       # data of all dumped arrays together; with the .npy headers the dump stays under 64 MB
+
+
+def _dump_outputs(dirname, arrays):
+    """Write {name: tensor or array} as dirname/<name>.npy, float32 (float64 where the output is float64).  The smallest arrays are
+    written whole; an array larger than its share of DUMP_BYTES is replaced by a sample of its flattened elements at positions drawn
+    from a generator seeded with 0 (sorted; the same positions for the same shape in every run)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    items = sorted(((k, np.asarray(v.detach().cpu() if hasattr(v, 'detach') else v)) for k, v in arrays.items()), key=lambda kv: kv[1].size)
+    left = DUMP_BYTES
+    for i, (name, a) in enumerate(items):
+        dtype = np.float64 if a.dtype == np.float64 else np.float32
+        n = left // (len(items) - i) // np.dtype(dtype).itemsize
+        if a.size > n:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).integers(0, a.size, n))]
+        a = a.astype(dtype)
+        np.save(os.path.join(dirname, name + '.npy'), a)
+        left -= a.nbytes
 
 
 def _traffic(kernel):
@@ -183,7 +206,7 @@ def run_reference(args):
             from next3d_b200 import drivers
             planes = og.synthesis(sd, cfg, ws, c_cam, v, u_c, u_f, return_intermediates=True)['planes']
             pts = drivers.create_samples(256, 1.0, head=256 ** 3 // 2, count=64 ** 3)
-            step = lambda: orr.run_model(sd, planes, pts, cfg.rendering_kwargs)
+            step = lambda: dict(zip(('rgb', 'sigma'), orr.run_model(sd, planes, pts, cfg.rendering_kwargs)))
             units_per_step, unit = (64 ** 3) / (256 ** 3), 'grids/s'
             sample = 'each step = 64^3 consecutive voxels (1/64) of the 256^3 grid through run_model (tri-plane fetch + decoder), planes precomputed'
         else:
@@ -194,8 +217,10 @@ def run_reference(args):
             step()
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            step()
+            out = step()
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        _dump_outputs(args.dump_outputs, out)
     val = args.steps * units_per_step / dt
     desc = f'{args.steps} steps, fp32 torch CPU ops (oracle port of the reference path), {cores} threads (of {os.cpu_count()} host cores; more threads are slower, see bench.py::_cpu_threads); {sample}'
     _emit({
@@ -299,7 +324,7 @@ def _kernel_profile(G, eng, ws_d, c_d, v_d):
 
 
 def _time_c5(G, ws, v, steps, warmup):
-    """256^3 density grid from cached planes: (ms per grid, roofline dict)."""
+    """256^3 density grid from cached planes: (ms per grid, roofline dict, the grid of the last timed step)."""
     import torch
     from next3d_b200 import kernels as K
     eng = G._get_engine()
@@ -327,11 +352,12 @@ def _time_c5(G, ws, v, steps, warmup):
             'note': 'algorithmic FLOPs of the full 256^3 grid; the %d border voxels the script overwrites with -1000 are not decoded '
                     '(%.0f %% of the grid), so the executed FLOPs are lower' % (R ** 3 - interior, 100.0 * (1 - interior / R ** 3)),
             'limits': {'mufu_floor_ms': 1e3 * interior * 128 / (148 * 16 * 1.85e9), 'l1_wavefront_floor_ms': 1e3 * interior * 12 / (148 * 1.85e9)}}
-    return ms, roof
+    return ms, roof, out
 
 
 def _time_c4(G, dev, rank, world, steps, warmup):
-    """One 240-frame clip split over the ranks: seconds for the whole clip (max over ranks), frames."""
+    """One 240-frame clip split over the ranks: seconds for the whole clip (max over ranks), frames, whether the frames look sane,
+    and the clip of the last timed step (uint8 [F, 512, 512, 3] host tensor on rank 0, None elsewhere)."""
     import torch
     import torch.distributed as dist
     from next3d_b200 import drivers, weights, distributed as D
@@ -355,7 +381,7 @@ def _time_c4(G, dev, rank, world, steps, warmup):
         _barrier(dist, world, dev)
     dt = D.max_over_ranks(e0.elapsed_time(e1) / 1e3, dev) / steps
     ok = frames is None or (frames.shape == (F, 512, 512, 3) and int(frames.float().std()) > 0)
-    return dt, F, ok
+    return dt, F, ok, frames
 
 
 def run_ours(args):
@@ -384,9 +410,11 @@ def run_ours(args):
             sampler = ClockSampler(local) if rank == 0 else None
             if sampler:
                 sampler.start()
-            ms, roof = _time_c5(G, ws, v.to(dev), args.steps, args.warmup)
+            ms, roof, grid = _time_c5(G, ws, v.to(dev), args.steps, args.warmup)
             clocks = sampler.stop(scope='warm-up + timed region (same load)') if sampler else None
         ms = 1e3 * D.max_over_ranks(ms / 1e3, dev)
+        if rank == 0 and args.dump_outputs:
+            _dump_outputs(args.dump_outputs, {'sigma_grid': grid})
         if rank == 0:
             _emit({'metric': spec['metric'], 'value': world * 1e3 / ms, 'unit': 'grids/s', 'n_gpus': world, 'steps': args.steps, 'warmup': args.warmup,
                    'ms_per_step': ms, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'bf16x3 decoder (fp32 accumulate), f32 elsewhere',
@@ -401,10 +429,12 @@ def run_ours(args):
         sampler = ClockSampler(local) if rank == 0 else None
         if sampler:
             sampler.start()
-        dt, F, ok = _time_c4(G, dev, rank, world, max(1, min(args.steps, 3)), args.warmup)
+        dt, F, ok, frames = _time_c4(G, dev, rank, world, args.steps, args.warmup)
         clocks = sampler.stop(scope='warm-up + timed region (same load)') if sampler else None
+        if rank == 0 and args.dump_outputs:
+            _dump_outputs(args.dump_outputs, {'frames': frames})
         if rank == 0:
-            _emit({'metric': spec['metric'], 'value': F / dt, 'unit': UNIT, 'n_gpus': world, 'steps': max(1, min(args.steps, 3)), 'warmup': args.warmup,
+            _emit({'metric': spec['metric'], 'value': F / dt, 'unit': UNIT, 'n_gpus': world, 'steps': args.steps, 'warmup': args.warmup,
                    'ms_per_step': 1e3 * dt, 'higher_is_better': True, 'scaling': 'strong', 'vs_baseline': None,
                    'dtype': 'bf16x3 (hi/lo split operands, fp32 accumulate) for convs; f32 elsewhere', 'data': 'synthetic',
                    'config': {'workload': spec['workload'] + f'batches of {spec["batch"]} frames per GPU', 'frames': F,
@@ -414,7 +444,7 @@ def run_ours(args):
                    'e2e': {'value': F / dt, 'unit': UNIT, 'h2d_bytes_per_step': int(F * (28 * 512 + 25) * 4),
                            'd2h_bytes_per_step': int(F * 512 * 512 * 3), 'ms_per_step': 1e3 * dt,
                            'note': 'this configuration IS end to end: host schedule -> H2D per batch -> synthesis -> uint8 -> gather -> D2H'},
-                   'gpu_launches': G._get_engine().launches * -(-F // (spec['batch'] * world)) * max(1, min(args.steps, 3))})
+                   'gpu_launches': G._get_engine().launches * -(-F // (spec['batch'] * world)) * args.steps})
         if world > 1:
             dist.destroy_process_group()
         return
@@ -498,13 +528,15 @@ def run_ours(args):
         t_begin = time.perf_counter()
         e0.record()
         for i in range(args.steps):
-            step_device(i)
+            out = step_device(i)
         if world > 1:
             torch.cuda.current_stream(dev).wait_stream(side)
         e1.record()
         _barrier(dist, world, dev)
         t_end = time.perf_counter()
         dt = D.max_over_ranks(e0.elapsed_time(e1) / 1e3, dev)
+        if rank == 0 and args.dump_outputs:                    # before the loops below overwrite the graph's static outputs
+            _dump_outputs(args.dump_outputs, out)
         gather_ms = statistics.median([x.elapsed_time(y) for x, y in gather_ev]) if gather_ev else None
 
         # ---- end to end through the public API: pinned host inputs -> synthesis -> images on the host
@@ -552,7 +584,7 @@ def run_ours(args):
         if rank == 0 and world == 1 and name == 'c2' and not args.no_other_configs:
             others = {}
             try:
-                ms5, roof5 = _time_c5(G, ws_d, v_d, 5, 2)
+                ms5, roof5, _ = _time_c5(G, ws_d, v_d, 5, 2)
                 others['c5'] = {'metric': CONFIGS['c5']['metric'], 'value': 1e3 / ms5, 'unit': 'grids/s', 'ms_per_step': ms5, 'steps': 5,
                                 'config': {'workload': CONFIGS['c5']['workload'] + 'one GPU'}, 'roofline': roof5}
             except Exception as e:                                              # an extra must never take the headline down
@@ -589,7 +621,7 @@ def run_ours(args):
                                         'config': {'workload': CONFIGS['c3']['workload'] + f'batch {B3}, one GPU', 'global_batch': B3},
                                         'roofline_renderer': roof3}
                     else:
-                        dt4, F4, ok4 = _time_c4(G2, dev, 0, 1, 1, 1)
+                        dt4, F4, ok4, _ = _time_c4(G2, dev, 0, 1, 1, 1)
                         others['c4'] = {'metric': CONFIGS['c4']['metric'], 'value': F4 / dt4, 'unit': UNIT, 'ms_per_step': 1e3 * dt4, 'steps': 1,
                                         'config': {'workload': CONFIGS['c4']['workload'] + 'one GPU', 'frames': F4}, 'frames_ok': ok4, 'scaling': 'strong'}
                     del G2
@@ -638,6 +670,8 @@ def main():
     ap.add_argument('--no-other-configs', action='store_true', help='default N=1 run: skip the short c3 / c4 / c5 runs')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='launch kernels eagerly instead of replaying the captured CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)')
     args = ap.parse_args()
     _guard_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup

@@ -10,9 +10,8 @@ This module installs sys.modules stubs for those, plugs OUR CPU rasterizer resta
 (oracle/rasterize.py, pytorch3d semantics per SURVEY.md Appendix C) in place of pytorch3d, writes
 a synthetic eye mask into a scratch cwd, and returns the reference's own TriPlaneGenerator.
 
-It is used ONLY by tests/golden/make_golden.py and tests/test_oracle_vs_reference.py to pin the
-oracle restatement against the reference's own code; /root/reference does not exist on the GPU
-box, so nothing that runs there imports this file.
+It is used ONLY by tests/golden/make_golden.py, which stores what the reference's own code returns
+so that the tests pin the oracle restatement against it without a checkout of the reference.
 """
 import os
 import sys

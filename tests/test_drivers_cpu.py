@@ -1,39 +1,32 @@
 """Row f1 of SURVEY.md section 8 (batched frame drivers): the frame schedule and the batching logic against the reference's own
-per-frame code (gen_videos_next3d.py:96-171, camera_utils.py:68-86).  CPU only; the generator is a stub here, the real one is
-covered by tests/test_gpu_generator.py (batch invariance)."""
-import math
-import os
-import sys
-
+per-frame code (gen_videos_next3d.py:96-171, camera_utils.py:68-86), through what that code returned for the same inputs
+(tests/golden/reference_checks.npz, written by tests/golden/make_golden.py).  CPU only; the generator is a stub here, the real one
+is covered by tests/test_gpu_generator.py (batch invariance)."""
 import numpy as np
 import pytest
 import torch
 
 from next3d_b200 import camera, drivers
+from tests.golden.make_golden import CAMERA_VIEWS, ORBIT_FRAMES, grid_sample_index, grid_slices, key
+from tests.helpers import load_golden
 
-REF = '/root/reference'
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, 'camera_utils.py')), reason='reference tree not present (GPU box)')
+
+@pytest.fixture(scope='module')
+def ref():
+    return {k: torch.from_numpy(v) for k, v in load_golden('reference_checks').items()}
 
 
-@needs_ref
-def test_cameras_match_reference_sampler():
-    sys.path.insert(0, REF)
-    try:
-        import camera_utils
-    finally:
-        sys.path.remove(REF)
+def test_cameras_match_reference_sampler(ref):
     lookat = torch.tensor([0, 0, 0.2])
-    for h, v in [(math.pi / 2, math.pi / 2), (math.pi / 2 + 0.4, math.pi / 2 - 0.2), (0.3, 1e-7), (3.0, 3.2)]:
-        ref = camera_utils.LookAtPoseSampler.sample(h, v, lookat, radius=2.7)[0]
-        assert torch.equal(camera.look_at_pose(h, v, lookat, 2.7), ref)
-    assert torch.equal(camera.fov_to_intrinsics(18.837), camera_utils.FOV_to_intrinsics(18.837))
+    for i, (h, v) in enumerate(CAMERA_VIEWS):
+        assert torch.equal(camera.look_at_pose(h, v, lookat, 2.7), ref[key('look_at', i)])
+    assert torch.equal(camera.fov_to_intrinsics(18.837), ref['fov_intrinsics'])
     # the orbit of gen_videos_next3d.py:128-140, frame by frame
-    F = 24
+    F = ORBIT_FRAMES
     c = drivers.orbit_camera_params(F, lookat, 2.7)
     intr = torch.tensor([[4.2647, 0, 0.5], [0, 4.2647, 0.5], [0, 0, 1]])
     for f in range(F):
-        pose = camera_utils.LookAtPoseSampler.sample(3.14 / 2 + 0.35 * np.sin(2 * 3.14 * f / (F // 2)),
-                                                      3.14 / 2 - 0.05 + 0.25 * np.cos(2 * 3.14 * f / (F // 2)), lookat, radius=2.7)
+        pose = ref['orbit_poses'][f:f + 1]
         assert torch.equal(c[f], torch.cat([pose.reshape(-1, 16), intr.reshape(-1, 9)], 1)[0])
 
 
@@ -50,14 +43,11 @@ def test_interpolated_latents_match_per_frame_calls():
     assert np.allclose(got[::w_frames].numpy(), ws.numpy(), atol=1e-6)    # passes through the key frames
 
 
-@needs_ref
-def test_uint8_conversion_is_layout_grid():
-    layout_grid = _reference_scripts()[1].layout_grid                      # gen_videos_next3d.py:35-49
-    g = torch.Generator().manual_seed(1)
-    img = torch.randn(2, 3, 8, 8, generator=g) * 1.5
+def test_uint8_conversion_is_layout_grid(ref):
+    img = ref['layout_grid_x']
     got = drivers.to_uint8_hwc(img)
     for k in range(2):
-        assert np.array_equal(got[k].numpy(), layout_grid(img[k:k + 1], grid_w=1, grid_h=1))
+        assert np.array_equal(got[k].numpy(), ref['layout_grid'][k].numpy())     # gen_videos_next3d.py:35-49, one image per grid
 
 
 class _StubG(torch.nn.Module):
@@ -92,24 +82,16 @@ def test_batched_frames_equal_per_frame_loop(F, batch, mesh):
 
 
 # ------------------------------------------------------------------------------------------------ row f2: shape extraction
-def _reference_scripts():
-    """The reference's own gen_samples_next3d / gen_videos_next3d modules (through the oracle's import shims)."""
-    from oracle import ref_shim
-    ref_shim.import_reference()
-    with ref_shim.in_scratch():
-        import gen_samples_next3d
-        import gen_videos_next3d
-    return gen_samples_next3d, gen_videos_next3d
-
-
-@needs_ref
 @pytest.mark.parametrize('N', [17, 64])
-def test_chunked_samples_are_slices_of_the_reference_grid(N):
-    ref = _reference_scripts()[0].create_samples(N=N, voxel_origin=[0, 0, 0], cube_length=1.0)[0]
-    assert torch.equal(drivers.create_samples(N, 1.0), ref)
-    for head, n in [(0, 1000), (N ** 3 - 777, 777), (12345 % N ** 3, 2048)]:
-        n = min(n, N ** 3 - head)
-        assert torch.equal(drivers.create_samples(N, 1.0, head, n), ref[:, head:head + n])
+def test_chunked_samples_are_slices_of_the_reference_grid(ref, N):
+    """gen_samples_next3d.create_samples, stored at the points make_golden.grid_sample_index lists: the whole 17^3 grid, and
+    every 61st point of the 64^3 grid plus the chunks checked below."""
+    idx = torch.from_numpy(grid_sample_index(N))
+    grid = ref[key('create_samples', N)]
+    assert torch.equal(drivers.create_samples(N, 1.0)[:, idx], grid)
+    for head, n in grid_slices(N):
+        pos = torch.searchsorted(idx, torch.arange(head, head + n))
+        assert torch.equal(drivers.create_samples(N, 1.0, head, n), grid[:, pos])
 
 
 def test_large_index_rounding_like_the_reference():

@@ -1,5 +1,6 @@
 """Row f3 of SURVEY.md section 8: native .obj / landmark parsers vs the reference's own parsing code (gen_samples_next3d.py:165-178,
 restated below as the oracle), bit-exact in float32.  CPU only."""
+import gzip
 import os
 
 import numpy as np
@@ -7,8 +8,7 @@ import pytest
 import torch
 
 from next3d_b200 import inputs
-
-REF_DEMO = '/root/reference/data/demo'
+from tests.helpers import GOLDEN_DIR
 
 
 def ref_parse_obj(path):
@@ -45,9 +45,12 @@ def test_obj_vertices_bit_exact(tmp_path):
     assert np.array_equal(inputs.load_obj_vertices(open(p, 'rb').read()).view(np.uint32), ref.view(np.uint32))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_DEMO), reason='reference demo assets not present (GPU box)')
-def test_reference_demo_frame():
-    obj, lms = os.path.join(REF_DEMO, 'demo.obj'), os.path.join(REF_DEMO, 'demo_kpt2d.txt')
+def test_reference_demo_frame(tmp_path):
+    """The reference's demo FLAME frame (data/demo/demo.obj, stored gzipped, and data/demo/demo_kpt2d.txt)."""
+    obj, lms = tmp_path / 'demo.obj', os.path.join(GOLDEN_DIR, 'demo_kpt2d.txt')
+    with gzip.open(os.path.join(GOLDEN_DIR, 'demo.obj.gz'), 'rb') as f:
+        obj.write_bytes(f.read())
+    obj = str(obj)
     v = ref_parse_obj(obj)
     l = torch.from_numpy(np.loadtxt(lms)).float().unsqueeze(0)
     ref = torch.cat((v, l), 1)                                            # gen_samples_next3d.py:176-178

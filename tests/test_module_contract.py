@@ -1,9 +1,13 @@
 """CPU: the drop-in TriPlaneGenerator keeps the reference's state-dict contract and API, and refuses to run on CPU."""
+import json
+import os
+
 import pytest
 import torch
 
 from next3d_b200 import config, weights
-from oracle import generator as og, ref_shim
+from oracle import generator as og
+from tests.helpers import GOLDEN_DIR
 
 
 def _tiny():
@@ -40,16 +44,18 @@ def test_no_cpu_fallback():
         G.synthesis(ws, c_cam, v, noise_mode='const')
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present')
 def test_reference_state_dict_round_trip():
-    """The reference's own loader path: copy_params_and_buffers(G_ref, G_new, require_all=True) (gen_samples_next3d.py:153)."""
+    """The reference's own loader path: copy_params_and_buffers(G_ref, G_new, require_all=True) (gen_samples_next3d.py:153), then
+    G_new.load_state_dict(G_ref.state_dict()), against the names and shapes the reference's TriPlaneGenerator of the same config
+    reports (tests/golden/reference_state_dict.json, written by tests/golden/make_golden.py)."""
     cfg, sd, G = _tiny()
-    G_ref = ref_shim.build_reference_generator(cfg)
-    G_ref.load_state_dict(sd)
-    from torch_utils import misc
-    misc.copy_params_and_buffers(G_ref, G, require_all=True)
-    G.load_state_dict(G_ref.state_dict())
-    assert set(G.state_dict().keys()) == set(G_ref.state_dict().keys())
+    with open(os.path.join(GOLDEN_DIR, 'reference_state_dict.json')) as f:
+        ref = {k: {n: tuple(shape) for n, shape in v} for k, v in json.load(f).items()}
+    for name, t in list(G.named_parameters()) + list(G.named_buffers()):      # misc.copy_params_and_buffers, require_all=True
+        assert name in ref['params_and_buffers'], name
+        assert tuple(t.shape) == ref['params_and_buffers'][name], name
+    assert {n: tuple(t.shape) for n, t in G.state_dict().items()} == ref['state_dict']
+    G.load_state_dict({n: sd[n] for n in ref['state_dict']})
 
 
 def test_engine_cache_key_tracks_weights_mask_and_options():
