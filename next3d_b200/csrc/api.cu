@@ -31,3 +31,14 @@ N3DDeviceState* n3d_device_state(void) {
     }
     return d;
 }
+
+int n3d_smem_optin(N3DDeviceState* D, unsigned cfg_bit, const void* kernel, int bytes, const char* who) {
+    if (D->configured & cfg_bit) return N3D_OK;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e != cudaSuccess) {
+        n3d_set_error("%s: cannot raise dynamic shared memory to %d bytes: %s", who, bytes, cudaGetErrorString(e));
+        return N3D_ERR_CUDA;
+    }
+    D->configured |= cfg_bit;
+    return N3D_OK;
+}

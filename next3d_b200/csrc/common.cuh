@@ -39,8 +39,12 @@ struct N3DDeviceState {
     int num_sms;
     unsigned configured;     // bit per kernel, see N3D_CFG_*
 };
-enum { N3D_CFG_CONV = 1u, N3D_CFG_FILL_MOUTH = 2u, N3D_CFG_RENDER16 = 4u, N3D_CFG_RENDER32 = 8u, N3D_CFG_POINTS = 16u, N3D_CFG_FIR_STREAM = 32u, N3D_CFG_FIR_DOWN_STREAM = 64u };
+enum { N3D_CFG_CONV = 1u, N3D_CFG_FILL_MOUTH = 2u, N3D_CFG_RENDER16 = 4u, N3D_CFG_RENDER32 = 8u, N3D_CFG_POINTS = 16u, N3D_CFG_FIR_STREAM = 32u, N3D_CFG_FIR_DOWN_STREAM = 64u,
+       N3D_CFG_POINTS_RGB = 128u, N3D_CFG_FLOOR_GATHER = 256u };
 N3DDeviceState* n3d_device_state(void);      // api.cu; nullptr (+ error message) when the current device cannot be queried
+// api.cu: raises `kernel`'s dynamic shared-memory limit to `bytes` once per device (bit `cfg_bit` of D->configured).  N3D_OK, or
+// N3D_ERR_CUDA with an error message naming `who`.
+int n3d_smem_optin(N3DDeviceState* D, unsigned cfg_bit, const void* kernel, int bytes, const char* who);
 
 // fp32 -> (hi, lo) bf16 pair with hi + lo ~= x to ~16 mantissa bits (used by the 3-product tensor-core scheme).
 __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {

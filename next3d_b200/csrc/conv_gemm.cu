@@ -567,13 +567,7 @@ int launch_conv(const N3DConvGemm* p, int nsub, const SubSpec* specs, void* stre
     const int smem = K.stages * K.stage_bytes + 8 * (2 * K.stages + 4) + 32 + 2 * kStageArrays * kMaxBlockN * 4 + 1024;
     N3DDeviceState* D = n3d_device_state();
     if (!D) return N3D_ERR_CUDA;
-    if (!(D->configured & N3D_CFG_CONV)) {
-        if (cudaFuncSetAttribute(conv_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
-            n3d_set_error("n3d_conv_gemm: cannot raise dynamic shared memory to 227 KiB");
-            return N3D_ERR_CUDA;
-        }
-        D->configured |= N3D_CFG_CONV;
-    }
+    if (int e = n3d_smem_optin(D, N3D_CFG_CONV, (const void*)conv_gemm_kernel, 227 * 1024, "n3d_conv_gemm")) return e;
     const int total_tiles = tiles_m * K.tiles_n * splits;
     const int num_sms = D->num_sms;
     const int grid = min(total_tiles, num_sms);

@@ -176,200 +176,239 @@ __device__ __forceinline__ void epi_store(const EpiParams& E, const EpiVec& V, c
     }
 }
 
-// Horizontal pass of the separable 4-tap FIR for one raw row: the NC outputs that start at columns xs .. xs+NC-1 (NC + 3 float4
-// loads at p, p + cs, ...; only the first / last column can fall outside the image: flags vl / vr).  `p` is null for a row outside
-// the image (zero padding).
-template <int NC>
-__device__ __forceinline__ void fir_hrow(const float4* __restrict__ p, int cs, bool vl, bool vr, const float (&g)[4], float4 (&h)[NC]) {
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-    for (int b = 0; b < NC; ++b) h[b] = z;
-    if (!p) return;
-    float4 v[NC + 3];
-    v[0] = vl ? __ldg(p) : z;
-#pragma unroll
-    for (int c = 1; c < NC + 2; ++c) v[c] = __ldg(p + c * cs);
-    v[NC + 2] = vr ? __ldg(p + (NC + 2) * cs) : z;
-#pragma unroll
-    for (int b = 0; b < NC; ++b) {
-        h[b] = f4_scale(g[0], v[b]);
-#pragma unroll
-        for (int fx = 1; fx < 4; ++fx) h[b] = f4_fma(g[fx], v[b + fx], h[b]);
-    }
+// ---------------------------------------------------------------------------------------------- FIR passes
+// Both FIR passes (up: after every up-conv, with the epilogue; down: before every stride-2 conv) evaluate the separable 4x4 FIR one
+// 2x2 output block and one 4-channel group per thread: a horizontal pass over the raw rows of a five-column window, then a vertical
+// pass over five filtered rows.  Consecutive blocks down a column share 3 of the 5 rows, so the filtered rows stay in registers and
+// slide down: 2 row reads per block instead of 5 (the unshared form is bound by L2->L1 traffic, 2.5x the raw tensor).
+// Each direction has a register-tiled kernel (rows read from global memory) and a streamed one (rows read from a shared-memory ring
+// filled by bulk copies).  Both call the functions below for every arithmetic instruction, so they round identically and the
+// batch-size-dependent choice between them never shows in the results.
+
+// 1-D taps [1, 3, 3, 1] * s: s = 1/4 for up (upfirdn2d's gain 4 spread over both axes), 1/8 for down.
+constexpr float kFirUpS = 0.25f, kFirDownS = 0.125f;
+
+__device__ __forceinline__ float4 fir4(float s, const float4& a, const float4& b, const float4& c, const float4& d) {
+    return f4_fma(s, d, f4_fma(3.f * s, c, f4_fma(3.f * s, b, f4_scale(s, a))));
 }
 
-// thread = (image, strip of S vertically adjacent output row pairs, NC output columns, 4-channel group).  The 4x4 FIR is separable
-// ([1,3,3,1]/8 * 2 per axis).  A 2 x NC output block needs 5 raw rows x (NC + 3) raw columns; consecutive blocks of the strip share
-// 3 of the 5 rows, so the horizontally filtered rows are kept in registers and slid down the strip: 2 (NC + 3) float4 loads per
-// 2 NC outputs instead of 5 (NC + 3) (the unshared form is bound by L2->L1 traffic, 2.5x the raw tensor).
-template <int NC>
+// Horizontal pass over raw row r: the two outputs that start at window columns 0 and 1.  A window column with ok[q] == false lies
+// outside the image and reads as zero; so does a row outside [0, src.rows).  `Src` is where the rows come from (GlobalRows, RowRing).
+template <class Src>
+__device__ __forceinline__ void fir_hrow(Src& src, int r, float s, const bool (&ok)[5], float4 (&h)[2]) {
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    h[0] = z; h[1] = z;
+    if (r < 0 || r >= src.rows) return;
+    const float4* p = src.acquire(r);
+    float4 v[5];
+#pragma unroll
+    for (int q = 0; q < 5; ++q) v[q] = ok[q] ? src.ld(p, q) : z;
+    h[0] = fir4(s, v[0], v[1], v[2], v[3]);
+    h[1] = fir4(s, v[1], v[2], v[3], v[4]);
+    src.release();
+}
+
+// Up: window = raw columns x0-1 .. x0+3 of the 2-column block at x0; only the first / last can fall outside the image (vl / vr).
+template <class Src>
+__device__ __forceinline__ void fir_hrow_up(Src& src, int r, bool vl, bool vr, float4 (&h)[2]) {
+    fir_hrow(src, r, kFirUpS, {vl, true, true, true, vr}, h);
+}
+
+// Down: window = input columns x0-2 .. x0+2, x0 even in [0, W]: the first two are outside together (x0 == 0: vl), the next two
+// together (x0 == W: vm), the last one when x0 + 2 >= W (vr).
+template <class Src>
+__device__ __forceinline__ void fir_hrow_down(Src& src, int r, bool vl, bool vm, bool vr, float4 (&h)[2]) {
+    fir_hrow(src, r, kFirDownS, {vl, vl, vm, vm, vr}, h);
+}
+
+// Vertical pass of output row a, column b of the block from the filtered rows a .. a+3.
+__device__ __forceinline__ float4 fir_vert(float s, const float4 (&h)[5][2], int a, int b) {
+    return fir4(s, h[a][b], h[a + 1][b], h[a + 2][b], h[a + 3][b]);
+}
+
+// The window moves down two rows: filtered rows 2 .. 4 become rows 0 .. 2.
+__device__ __forceinline__ void fir_slide(float4 (&h)[5][2]) {
+#pragma unroll
+    for (int r = 0; r < 3; ++r) { h[r][0] = h[r + 2][0]; h[r][1] = h[r + 2][1]; }
+}
+
+// Raw noise of the 2x2 block at (y0, x0) of an image's [H2, W2] noise plane nzp (null: no noise), as {(0,0), (0,1), (1,0), (1,1)}.
+__device__ __forceinline__ float4 fir_up_noise(const float* nzp, int y0, int W2) {
+    if (!nzp) return make_float4(0.f, 0.f, 0.f, 0.f);
+    const float* p = nzp + (int64_t)y0 * W2;
+    return make_float4(__ldg(p), __ldg(p + 1), __ldg(p + W2), __ldg(p + W2 + 1));
+}
+
+// One step of the FIR-up epilogue: the 2x2 output block at cursor P from the filtered rows h and its raw noise nz, then window and
+// cursor move down two rows.
+__device__ __forceinline__ void fir_up_block(const EpiParams& E, const EpiVec& V, EpiCursor& P, int W2, float4 nz, float4 (&h)[5][2]) {
+    // explicit: no FMA contraction into the bias add
+    const float nzg[4] = {__fmul_rn(E.gain, nz.x), __fmul_rn(E.gain, nz.y), __fmul_rn(E.gain, nz.z), __fmul_rn(E.gain, nz.w)};
+#pragma unroll
+    for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b) epi_store(E, V, P, fir_vert(kFirUpS, h, a, b), nzg[2 * a + b], a * W2 + b);
+    fir_slide(h);
+    P.f32 += 2 * (int64_t)W2 * E.f32_cstride;
+    P.sp[0] += 2 * (int64_t)W2 * E.out[0].cstride;
+    P.sp[1] += 2 * (int64_t)W2 * E.out[1].cstride;
+}
+
+// One step of the FIR-down pass: the 2x2 FIR outputs (y0 + a, x0 + b) of one sub-pixel, zero beyond the (H+1)x(W+1) FIR output, as
+// bf16 hi / lo into parity image a * 2 + b (hi, lo: the sub-pixel in parity image 0), written only when `active`; then the window
+// moves down two rows.
+__device__ __forceinline__ void fir_down_block(float4 (&h)[5][2], bool active, int y0, int x0, int H, int W, int64_t par_stride,
+                                               __nv_bfloat16* hi, __nv_bfloat16* lo) {
+    if (active) {
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int b = 0; b < 2; ++b) {
+                float4 v = fir_vert(kFirDownS, h, a, b);
+                if (y0 + a > H || x0 + b > W) v = make_float4(0.f, 0.f, 0.f, 0.f);
+                uint2 hh, l;
+                split_bf16x2(v.x, v.y, hh.x, l.x); split_bf16x2(v.z, v.w, hh.y, l.y);
+                const int64_t off = (int64_t)(a * 2 + b) * par_stride;
+                *reinterpret_cast<uint2*>(hi + off) = hh;
+                *reinterpret_cast<uint2*>(lo + off) = l;
+            }
+    }
+    fir_slide(h);
+}
+
+// Raw rows of the register-tiled kernels, read from global memory on the read-only path.  col: the thread's first window column in
+// row 0; stride, cs: row and column stride in float4; rows: image height.
+struct GlobalRows {
+    const float4* col; int64_t stride; int rows, cs;
+    __device__ const float4* acquire(int r) const { return col + r * stride; }
+    __device__ float4 ld(const float4* p, int q) const { return __ldg(p + q * cs); }
+    __device__ void release() const {}
+};
+
+// Raw rows of the streamed kernels.  A CTA's tile needs a window of ncols raw columns of one image; a producer lane streams the
+// window's rows -- each a CONTIGUOUS ncols * C * 4-byte segment of the NHWC tensor -- through NR shared-memory stages with 1-D
+// bulk copies (TMA engine, mbarrier full / empty pair per stage), and the kFsConsumers consumer threads read their five columns from
+// the stages.  Loads are in flight NR rows ahead of the arithmetic and cost no registers.  Each thread counts its own stage / phase.
+constexpr int kFsConsumers = 256, kFsThreads = kFsConsumers + 32;
+constexpr int kFsSmemLimit = 112 * 1024;          // dynamic shared memory limit of both streamed kernels: 2 CTAs per SM
+
+struct RowRing {
+    int NR, rows, ncols, c4n;      // rows: image height; rows outside [0, rows) are zero padding, neither copied nor waited for
+    const float4* win;             // consumers: the thread's first window column in stage 0
+    uint32_t ring, bars;           // shared addresses: NR stages of ncols * c4n float4, then NR full and NR empty barriers
+    int s = 0; uint32_t ph = 0;
+
+    // smem: the CTA's dynamic shared memory; off: float4 offset of the thread's first window column within a stage
+    __device__ RowRing(uint8_t* smem, int NR, int rows, int ncols, int c4n, int off)
+        : NR(NR), rows(rows), ncols(ncols), c4n(c4n), win(reinterpret_cast<const float4*>(smem) + off), ring(n3d_tc::smem_u32(smem)),
+          bars(ring + (uint32_t)(NR * ncols * c4n) * 16u) {}
+    __device__ uint32_t stage(int k) const { return ring + (uint32_t)(k * ncols * c4n) * 16u; }
+    __device__ uint32_t full(int k) const { return bars + 8u * (uint32_t)k; }
+    __device__ uint32_t empty(int k) const { return bars + 8u * (uint32_t)(NR + k); }
+    __device__ void advance() { if (++s == NR) { s = 0; ph ^= 1u; } }
+
+    __device__ void init() const {          // every thread of the CTA
+        if (threadIdx.x == 0) {
+            for (int k = 0; k < NR; ++k) { n3d_tc::mbar_init(full(k), 1); n3d_tc::mbar_init(empty(k), kFsConsumers / 32); }
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+        __syncthreads();
+    }
+
+    // Producer lane: rows first .. last of the window that starts at column col0 of an image (img: its pixel (0, 0); `width` pixels
+    // per row), each clipped to the image's columns (the consumers' edge flags zero the clipped ones).
+    __device__ void produce(const float* img, int width, int col0, int first, int last) {
+        const int C = 4 * c4n;
+        const int col_lo = max(col0, 0), col_hi = min(col0 + ncols - 1, width - 1);
+        const uint32_t bytes = (uint32_t)(col_hi - col_lo + 1) * (uint32_t)C * 4u;
+        const uint32_t dst_off = (uint32_t)(col_lo - col0) * (uint32_t)C * 4u;
+        const float* src = img + (int64_t)col_lo * C;
+        for (int r = first; r <= last; ++r) {
+            if (r < 0 || r >= rows) continue;
+            n3d_tc::mbar_wait_short(empty(s), ph ^ 1u);
+            n3d_tc::mbar_expect_tx(full(s), bytes);
+            n3d_tc::bulk_load_1d(stage(s) + dst_off, src + (int64_t)r * width * C, bytes, full(s));
+            advance();
+        }
+    }
+
+    // Consumers (the row source of fir_hrow): wait for the next row's stage, read it, hand it back.
+    __device__ const float4* acquire(int) {
+        n3d_tc::mbar_wait_short(full(s), ph);
+        return win + s * ncols * c4n;
+    }
+    __device__ float4 ld(const float4* p, int q) const { return p[q * c4n]; }
+    __device__ void release() {
+        __syncwarp();                      // every lane has consumed its values: the stage may be refilled
+        if ((threadIdx.x & 31) == 0) n3d_tc::mbar_arrive(empty(s));
+        advance();
+    }
+};
+
+// FIR-up epilogue, register-tiled: thread = (image, strip of S output row pairs, 2 output columns, 4-channel group).  2 columns per
+// thread measured best on B200 (1 column: +23 % time despite 1.5x the occupancy, 4 columns: +15 %).
 __global__ void __launch_bounds__(256) fir_up_epilogue_kernel(const float* __restrict__ raw, int N, int H2, int W2, int C, int S, EpiParams E) {
-    const int RH = H2 + 1, RW = W2 + 1, c4n = C >> 2, BH = H2 >> 1, BW = W2 / NC, nstrip = (BH + S - 1) / S;
+    const int RH = H2 + 1, RW = W2 + 1, c4n = C >> 2, BH = H2 >> 1, BW = W2 >> 1, nstrip = (BH + S - 1) / S;
     const int64_t total = (int64_t)N * nstrip * BW * c4n;
-    const int64_t rstride = (int64_t)RW * c4n;                  // raw row stride in float4
-    const float g[4] = {0.25f, 0.75f, 0.75f, 0.25f};
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int c4 = (int)(i % c4n);
         int64_t t = i / c4n;
         const int bx = (int)(t % BW); t /= BW;
         const int st = (int)(t % nstrip);
         const int n = (int)(t / nstrip);
-        const int x0 = bx * NC, c0 = c4 * 4;
+        const int x0 = bx * 2, c0 = c4 * 4;
         const int by_begin = st * S, by_end = min(by_begin + S, BH);
-        const bool vl = x0 > 0, vr = x0 + NC + 1 < RW;         // raw columns x0-1 .. x0+NC+1
-        // float4 pointer to raw(n, row 0, column x0-1, c0); rows are addressed relative to it
-        const float4* col = reinterpret_cast<const float4*>(raw) + ((int64_t)n * RH * RW + (x0 - 1)) * c4n + c4;
-        auto rowp = [&](int ry) -> const float4* { return (ry >= 0 && ry < RH) ? col + ry * rstride : nullptr; };
+        const bool vl = x0 > 0, vr = x0 + 3 < RW;
+        GlobalRows rows{reinterpret_cast<const float4*>(raw) + ((int64_t)n * RH * RW + (x0 - 1)) * c4n + c4, (int64_t)RW * c4n, RH, c4n};
         const EpiVec V = epi_load(E, n, C, c0);
         const float* nzp = E.noise ? E.noise + (int64_t)n * E.noise_nstride + x0 : nullptr;
-        float4 h[5][NC];
+        float4 h[5][2];
 #pragma unroll
-        for (int r = 0; r < 3; ++r) fir_hrow<NC>(rowp(2 * by_begin - 1 + r), c4n, vl, vr, g, h[r]);
+        for (int r = 0; r < 3; ++r) fir_hrow_up(rows, 2 * by_begin - 1 + r, vl, vr, h[r]);
         EpiCursor P = epi_cursor(E, ((int64_t)n * H2 + 2 * by_begin) * W2 + x0, c0);
-        const int64_t adv_f32 = 2 * (int64_t)W2 * E.f32_cstride, adv0 = 2 * (int64_t)W2 * E.out[0].cstride, adv1 = 2 * (int64_t)W2 * E.out[1].cstride;
-        for (int by = by_begin; by < by_end; ++by, P.f32 += adv_f32, P.sp[0] += adv0, P.sp[1] += adv1) {
-            const int y0 = by * 2;
-            fir_hrow<NC>(rowp(y0 + 2), c4n, vl, vr, g, h[3]);
-            fir_hrow<NC>(rowp(y0 + 3), c4n, vl, vr, g, h[4]);
-            float nz[2][NC];
-#pragma unroll
-            for (int a = 0; a < 2; ++a)
-#pragma unroll
-                for (int b = 0; b < NC; ++b) nz[a][b] = nzp ? __fmul_rn(E.gain, __ldg(nzp + (int64_t)(y0 + a) * W2 + b)) : 0.f;   // explicit: no FMA contraction into the bias add
-#pragma unroll
-            for (int a = 0; a < 2; ++a)
-#pragma unroll
-                for (int b = 0; b < NC; ++b) {
-                    float4 acc = f4_scale(g[0], h[a][b]);
-#pragma unroll
-                    for (int r = 1; r < 4; ++r) acc = f4_fma(g[r], h[a + r][b], acc);
-                    epi_store(E, V, P, acc, nz[a][b], a * W2 + b);
-                }
-#pragma unroll
-            for (int r = 0; r < 3; ++r)
-#pragma unroll
-                for (int b = 0; b < NC; ++b) h[r][b] = h[r + 2][b];
+        for (int y0 = 2 * by_begin; y0 < 2 * by_end; y0 += 2) {
+            fir_hrow_up(rows, y0 + 2, vl, vr, h[3]);
+            fir_hrow_up(rows, y0 + 3, vl, vr, h[4]);
+            fir_up_block(E, V, P, W2, fir_up_noise(nzp, y0, W2), h);
         }
     }
 }
 
-// ---------------------------------------------------------------------------------------------- streamed FIR-up epilogue
-// Same arithmetic as fir_up_epilogue_kernel<2> (bit-identical results), different data movement.  The register-tiled kernel above is
-// bound by load latency at 16 warps/SM (DRAM 42-62 % of peak, profiles/r02_ncu_glue.txt): every strip step waits for its own ten
-// 16-byte loads.  Here a CTA owns a (TR output rows) x (TC output columns) x (all C channels) tile of one image and a producer
-// thread streams the raw rows it needs -- each a CONTIGUOUS (TC + 3) * C * 4-byte segment of the NHWC tensor -- through a ring of
-// shared-memory stages with 1-D bulk copies (TMA engine, mbarrier full / empty pairs); the eight consumer warps read the five
-// columns of their 2-column output block from shared memory.  Loads are in flight NR rows ahead of the arithmetic and cost no
-// registers.  thread = (column pair, 4-channel group): (TC / 2) * (C / 4) == 256.
-constexpr int kFsConsumers = 256, kFsThreads = kFsConsumers + 32;
-
+// FIR-up epilogue, streamed.  The register-tiled kernel is bound by load latency at 16 warps/SM (DRAM 42-62 % of peak,
+// profiles/r02_ncu_glue.txt): every strip step waits for its own ten 16-byte loads.  Here a CTA owns a (TR output rows) x (TC output
+// columns) x (all C channels) tile of one image and reads its raw rows through a RowRing.  thread = (column pair, 4-channel group):
+// (TC / 2) * (C / 4) == 256.
 __global__ void __launch_bounds__(kFsThreads, 2) fir_up_stream_kernel(const float* __restrict__ raw, int N, int H2, int W2, int C, int TC, int TR, int NR,
                                                                        EpiParams E) {
-    using namespace n3d_tc;
     extern __shared__ __align__(128) uint8_t fs_smem[];
     const int RH = H2 + 1, RW = W2 + 1, c4n = C >> 2;
-    const int row_f4 = (TC + 3) * c4n;                          // float4 per stage (one raw row segment)
-    const uint32_t row_bytes = (uint32_t)row_f4 * 16u;
-    const uint32_t ring = smem_u32(fs_smem), bars = ring + (uint32_t)NR * row_bytes;
-    auto full_bar = [&](int s) { return bars + 8u * (uint32_t)s; };
-    auto empty_bar = [&](int s) { return bars + 8u * (uint32_t)(NR + s); };
     const int tiles_x = W2 / TC, tiles_y = H2 / TR;
     const int bx = blockIdx.x % tiles_x, by = (blockIdx.x / tiles_x) % tiles_y, n = blockIdx.x / (tiles_x * tiles_y);
     const int X0 = bx * TC, Y0 = by * TR;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NR; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), kFsConsumers / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    if (warp == kFsConsumers / 32) {
-        // ===================================================== producer: raw rows Y0-1 .. Y0+TR+1, columns X0-1 .. X0+TC+1 (clipped)
-        if (lane == 0) {
-            const int col_lo = max(X0 - 1, 0), col_hi = min(X0 + TC + 1, RW - 1);
-            const uint32_t bytes = (uint32_t)(col_hi - col_lo + 1) * (uint32_t)C * 4u;
-            const uint32_t dst_off = (uint32_t)(col_lo - (X0 - 1)) * (uint32_t)C * 4u;
-            const float* src = raw + ((int64_t)n * RH * RW + col_lo) * C;
-            int s = 0; uint32_t ph = 0;
-            for (int ry = Y0 - 1; ry <= Y0 + TR + 1; ++ry) {
-                if (ry < 0 || ry >= RH) continue;               // zero padding: the consumers skip the same rows
-                mbar_wait_short(empty_bar(s), ph ^ 1u);
-                mbar_expect_tx(full_bar(s), bytes);
-                bulk_load_1d(ring + (uint32_t)s * row_bytes + dst_off, src + (int64_t)ry * RW * C, bytes, full_bar(s));
-                if (++s == NR) { s = 0; ph ^= 1u; }
-            }
-        }
+    const int c4 = threadIdx.x % c4n, j = threadIdx.x / c4n;
+    RowRing ring(fs_smem, NR, RH, TC + 3, c4n, 2 * j * c4n + c4);
+    ring.init();
+    if (threadIdx.x >= kFsConsumers) {      // producer: raw rows Y0-1 .. Y0+TR+1, columns X0-1 .. X0+TC+1
+        if (threadIdx.x == kFsConsumers) ring.produce(raw + (int64_t)n * RH * RW * C, RW, X0 - 1, Y0 - 1, Y0 + TR + 1);
         return;
     }
-
-    // ========================================================= consumers
-    const int c4 = threadIdx.x % c4n, j = threadIdx.x / c4n;
     const int x0 = X0 + 2 * j, c0 = c4 * 4;
-    const bool vl = x0 > 0, vr = x0 + 3 < RW;                   // raw columns x0-1 .. x0+3
-    const float4* base = reinterpret_cast<const float4*>(fs_smem) + (2 * j) * c4n + c4;
-    const float g[4] = {0.25f, 0.75f, 0.75f, 0.25f};
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    int s = 0; uint32_t ph = 0;
-    auto hrow = [&](int ry, float4 (&h)[2]) {
-        h[0] = z; h[1] = z;
-        if (ry < 0 || ry >= RH) return;
-        mbar_wait_short(full_bar(s), ph);
-        const float4* p = base + s * row_f4;
-        float4 v[5];
-        v[0] = vl ? p[0] : z;
-#pragma unroll
-        for (int q = 1; q < 4; ++q) v[q] = p[q * c4n];
-        v[4] = vr ? p[4 * c4n] : z;
-#pragma unroll
-        for (int b = 0; b < 2; ++b) {
-            h[b] = f4_scale(g[0], v[b]);
-#pragma unroll
-            for (int fx = 1; fx < 4; ++fx) h[b] = f4_fma(g[fx], v[b + fx], h[b]);
-        }
-        __syncwarp();                                           // every lane has consumed its values: the stage may be refilled
-        if (lane == 0) mbar_arrive(empty_bar(s));
-        if (++s == NR) { s = 0; ph ^= 1u; }
-    };
+    const bool vl = x0 > 0, vr = x0 + 3 < RW;
     const EpiVec V = epi_load(E, n, C, c0);
     const float* nzp = E.noise ? E.noise + (int64_t)n * E.noise_nstride + x0 : nullptr;
     float4 h[5][2];
 #pragma unroll
-    for (int r = 0; r < 3; ++r) hrow(Y0 - 1 + r, h[r]);
+    for (int r = 0; r < 3; ++r) fir_hrow_up(ring, Y0 - 1 + r, vl, vr, h[r]);
     EpiCursor P = epi_cursor(E, ((int64_t)n * H2 + Y0) * W2 + x0, c0);
-    const int64_t adv_f32 = 2 * (int64_t)W2 * E.f32_cstride, adv0 = 2 * (int64_t)W2 * E.out[0].cstride, adv1 = 2 * (int64_t)W2 * E.out[1].cstride;
-    // the noise of a 2x2 block is fetched one strip step ahead: its global-load latency was 26 % of all stall samples when it sat
-    // between the FIR and the stores (ncu source page of the first version)
-    float nzn[2][2];
-    auto load_noise = [&](int y0) {
-#pragma unroll
-        for (int a = 0; a < 2; ++a)
-#pragma unroll
-            for (int b = 0; b < 2; ++b) nzn[a][b] = nzp ? __ldg(nzp + (int64_t)(y0 + a) * W2 + b) : 0.f;
-    };
-    load_noise(Y0);
-    for (int y0 = Y0; y0 < Y0 + TR; y0 += 2, P.f32 += adv_f32, P.sp[0] += adv0, P.sp[1] += adv1) {
-        float nz[2][2];
-#pragma unroll
-        for (int a = 0; a < 2; ++a)
-#pragma unroll
-            for (int b = 0; b < 2; ++b) nz[a][b] = __fmul_rn(E.gain, nzn[a][b]);     // same rounding as the register-tiled kernel
-        if (y0 + 2 < Y0 + TR) load_noise(y0 + 2);
-        hrow(y0 + 2, h[3]);
-        hrow(y0 + 3, h[4]);
-#pragma unroll
-        for (int a = 0; a < 2; ++a)
-#pragma unroll
-            for (int b = 0; b < 2; ++b) {
-                float4 acc = f4_scale(g[0], h[a][b]);
-#pragma unroll
-                for (int r = 1; r < 4; ++r) acc = f4_fma(g[r], h[a + r][b], acc);
-                epi_store(E, V, P, acc, nz[a][b], a * W2 + b);
-            }
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-#pragma unroll
-            for (int b = 0; b < 2; ++b) h[r][b] = h[r + 2][b];
+    // the noise of a block is fetched one step ahead: its global-load latency was 26 % of all stall samples when it sat between the
+    // FIR and the stores (ncu source page of the first version)
+    float4 nz_next = fir_up_noise(nzp, Y0, W2);
+    for (int y0 = Y0; y0 < Y0 + TR; y0 += 2) {
+        const float4 nz = nz_next;
+        if (y0 + 2 < Y0 + TR) nz_next = fir_up_noise(nzp, y0 + 2, W2);
+        fir_hrow_up(ring, y0 + 2, vl, vr, h[3]);
+        fir_hrow_up(ring, y0 + 3, vl, vr, h[4]);
+        fir_up_block(E, V, P, W2, nz, h);
     }
 }
 
@@ -395,30 +434,14 @@ __global__ void __launch_bounds__(256) splitk_epilogue_kernel(const float* __res
     }
 }
 
-// Same for the down path, where the window starts two columns left of x0 (input columns x0-2 .. x0+2, x0 even in [0, W]): the
-// first two are outside together (x0 == 0: vl), the next two together (x0 == W: vm), the last one when x0 + 2 >= W (vr).
-__device__ __forceinline__ void fir_hrow_down(const float4* __restrict__ p, int cs, bool vl, bool vm, bool vr, const float (&g)[4], float4& h0, float4& h1) {
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    h0 = z; h1 = z;
-    if (!p) return;
-    float4 v[5];
-    v[0] = vl ? __ldg(p) : z; v[1] = vl ? __ldg(p + cs) : z;
-    v[2] = vm ? __ldg(p + 2 * cs) : z; v[3] = vm ? __ldg(p + 3 * cs) : z;
-    v[4] = vr ? __ldg(p + 4 * cs) : z;
-    h0 = f4_scale(g[0], v[0]); h1 = f4_scale(g[0], v[1]);
-#pragma unroll
-    for (int fx = 1; fx < 4; ++fx) { h0 = f4_fma(g[fx], v[fx], h0); h1 = f4_fma(g[fx], v[fx + 1], h1); }
-}
-
-// FIR (pad 2,2,2,2) -> [(H+1),(W+1)] -> parity-split bf16 hi/lo, layout [4 parities][N][SH][SW][C].
+// FIR (pad 2,2,2,2) -> [(H+1),(W+1)] -> parity-split bf16 hi/lo, layout [4 parities][N][SH][SW][C], register-tiled.
 // thread = (image, strip of S sub-pixel rows, sub-pixel column sx, 4-channel group) -> per sub-pixel the 2x2 block of FIR outputs
-// (2sy+a, 2sx+b), one per parity image; same register-resident sliding window over the horizontally filtered rows as above.
+// (2sy+a, 2sx+b), one per parity image.
 __global__ void __launch_bounds__(256) fir_down_split_kernel(const float* __restrict__ x, int N, int H, int W, int C, int S,
                                                              __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
     const int SH = (H + 2) / 2, SW = (W + 2) / 2, c4n = C >> 2, nstrip = (SH + S - 1) / S;
     const int64_t total = (int64_t)N * nstrip * SW * c4n;
     const int64_t par_stride = (int64_t)N * SH * SW * C;
-    const float g[4] = {0.125f, 0.375f, 0.375f, 0.125f};
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int c4 = (int)(i % c4n);
         int64_t t = i / c4n;
@@ -428,131 +451,50 @@ __global__ void __launch_bounds__(256) fir_down_split_kernel(const float* __rest
         const int x0 = sx * 2;                               // FIR output (y, x) reads input rows y-2 .. y+1, columns x-2 .. x+1
         const int sy_begin = st * S, sy_end = min(sy_begin + S, SH);
         const bool vl = x0 >= 2, vm = x0 < W, vr = x0 + 2 < W;
-        const float4* col = reinterpret_cast<const float4*>(x) + ((int64_t)n * H * W + (x0 - 2)) * c4n + c4;
-        const int64_t rstride = (int64_t)W * c4n;
-        auto rowp = [&](int iy) -> const float4* { return (iy >= 0 && iy < H) ? col + iy * rstride : nullptr; };
+        GlobalRows rows{reinterpret_cast<const float4*>(x) + ((int64_t)n * H * W + (x0 - 2)) * c4n + c4, (int64_t)W * c4n, H, c4n};
         float4 h[5][2];
 #pragma unroll
-        for (int r = 0; r < 3; ++r) fir_hrow_down(rowp(2 * sy_begin - 2 + r), c4n, vl, vm, vr, g, h[r][0], h[r][1]);
+        for (int r = 0; r < 3; ++r) fir_hrow_down(rows, 2 * sy_begin - 2 + r, vl, vm, vr, h[r]);
         for (int sy = sy_begin; sy < sy_end; ++sy) {
             const int y0 = sy * 2;
-            fir_hrow_down(rowp(y0 + 1), c4n, vl, vm, vr, g, h[3][0], h[3][1]);
-            fir_hrow_down(rowp(y0 + 2), c4n, vl, vm, vr, g, h[4][0], h[4][1]);
+            fir_hrow_down(rows, y0 + 1, vl, vm, vr, h[3]);
+            fir_hrow_down(rows, y0 + 2, vl, vm, vr, h[4]);
             const int64_t o = (((int64_t)n * SH + sy) * SW + sx) * C + c4 * 4;
-#pragma unroll
-            for (int a = 0; a < 2; ++a)
-#pragma unroll
-                for (int b = 0; b < 2; ++b) {
-                    float4 v = f4_scale(g[0], h[a][b]);
-#pragma unroll
-                    for (int r = 1; r < 4; ++r) v = f4_fma(g[r], h[a + r][b], v);
-                    if (y0 + a > H || x0 + b > W) v = make_float4(0.f, 0.f, 0.f, 0.f);     // beyond the (H+1)x(W+1) FIR output: zero pad
-                    uint2 hh, l;
-                    split_bf16x2(v.x, v.y, hh.x, l.x); split_bf16x2(v.z, v.w, hh.y, l.y);
-                    const int64_t off = (int64_t)(a * 2 + b) * par_stride + o;
-                    *reinterpret_cast<uint2*>(hi + off) = hh;
-                    *reinterpret_cast<uint2*>(lo + off) = l;
-                }
-#pragma unroll
-            for (int r = 0; r < 3; ++r) { h[r][0] = h[r + 2][0]; h[r][1] = h[r + 2][1]; }
+            fir_down_block(h, true, y0, x0, H, W, par_stride, hi + o, lo + o);
         }
     }
 }
 
-// Streamed form of fir_down_split_kernel (same arithmetic, bit-identical), built like fir_up_stream_kernel: a CTA owns TS sub-pixel rows x
-// TSC sub-pixel columns x all channels of one image ((TSC) * (C / 4) == 256 consumer threads) and a producer thread streams the
-// 2 TS + 3 input rows -- contiguous (2 TSC + 3) * C * 4-byte segments -- through the shared-memory ring with 1-D bulk copies.
+// FIR-down pass, streamed (same construction as fir_up_stream_kernel): a CTA owns TS sub-pixel rows x TSC sub-pixel columns x all
+// channels of one image ((TSC) * (C / 4) == 256 consumer threads) and reads its 2 TS + 3 input rows through a RowRing.
 __global__ void __launch_bounds__(kFsThreads, 2) fir_down_stream_kernel(const float* __restrict__ x, int N, int H, int W, int C, int TSC, int TS, int NR,
                                                                          __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
-    using namespace n3d_tc;
     extern __shared__ __align__(128) uint8_t fs_smem[];
     const int SH = (H + 2) / 2, SW = (W + 2) / 2, c4n = C >> 2;
-    const int row_f4 = (2 * TSC + 3) * c4n;
-    const uint32_t row_bytes = (uint32_t)row_f4 * 16u;
-    const uint32_t ring = smem_u32(fs_smem), bars = ring + (uint32_t)NR * row_bytes;
-    auto full_bar = [&](int s) { return bars + 8u * (uint32_t)s; };
-    auto empty_bar = [&](int s) { return bars + 8u * (uint32_t)(NR + s); };
     const int tiles_x = (SW + TSC - 1) / TSC, tiles_y = (SH + TS - 1) / TS;
     const int bx = blockIdx.x % tiles_x, by = (blockIdx.x / tiles_x) % tiles_y, n = blockIdx.x / (tiles_x * tiles_y);
     const int SX0 = bx * TSC, SY0 = by * TS, rows_here = min(TS, SH - SY0);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NR; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), kFsConsumers / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
     const int iy_first = 2 * SY0 - 2, iy_last = 2 * (SY0 + rows_here - 1) + 2;
-
-    if (warp == kFsConsumers / 32) {
-        if (lane == 0) {                                        // producer: input columns 2 SX0 - 2 .. 2 SX0 + 2 TSC, clipped to the image
-            const int col_lo = max(2 * SX0 - 2, 0), col_hi = min(2 * SX0 + 2 * TSC, W - 1);
-            const uint32_t bytes = (uint32_t)(col_hi - col_lo + 1) * (uint32_t)C * 4u;
-            const uint32_t dst_off = (uint32_t)(col_lo - (2 * SX0 - 2)) * (uint32_t)C * 4u;
-            const float* src = x + ((int64_t)n * H * W + col_lo) * C;
-            int s = 0; uint32_t ph = 0;
-            for (int iy = iy_first; iy <= iy_last; ++iy) {
-                if (iy < 0 || iy >= H) continue;
-                mbar_wait_short(empty_bar(s), ph ^ 1u);
-                mbar_expect_tx(full_bar(s), bytes);
-                bulk_load_1d(ring + (uint32_t)s * row_bytes + dst_off, src + (int64_t)iy * W * C, bytes, full_bar(s));
-                if (++s == NR) { s = 0; ph ^= 1u; }
-            }
-        }
+    const int c4 = threadIdx.x % c4n, j = threadIdx.x / c4n;
+    RowRing ring(fs_smem, NR, H, 2 * TSC + 3, c4n, 2 * j * c4n + c4);
+    ring.init();
+    if (threadIdx.x >= kFsConsumers) {      // producer: input columns 2 SX0 - 2 .. 2 SX0 + 2 TSC
+        if (threadIdx.x == kFsConsumers) ring.produce(x + (int64_t)n * H * W * C, W, 2 * SX0 - 2, iy_first, iy_last);
         return;
     }
-
-    const int c4 = threadIdx.x % c4n, j = threadIdx.x / c4n;
     const int sx = SX0 + j, x0 = 2 * sx;
     const bool active = sx < SW;                                // the last column tile is ragged (SW = W / 2 + 1)
     const bool vl = active && x0 >= 2, vm = active && x0 < W, vr = active && x0 + 2 < W;
-    const float4* base = reinterpret_cast<const float4*>(fs_smem) + (2 * j) * c4n + c4;      // input column x0 - 2
-    const float g[4] = {0.125f, 0.375f, 0.375f, 0.125f};
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    int s = 0; uint32_t ph = 0;
-    auto hrow = [&](int iy, float4& h0, float4& h1) {
-        h0 = z; h1 = z;
-        if (iy < 0 || iy >= H) return;
-        mbar_wait_short(full_bar(s), ph);
-        const float4* p = base + s * row_f4;
-        float4 v[5];
-        v[0] = vl ? p[0] : z; v[1] = vl ? p[c4n] : z;
-        v[2] = vm ? p[2 * c4n] : z; v[3] = vm ? p[3 * c4n] : z;
-        v[4] = vr ? p[4 * c4n] : z;
-        h0 = f4_scale(g[0], v[0]); h1 = f4_scale(g[0], v[1]);
-#pragma unroll
-        for (int fx = 1; fx < 4; ++fx) { h0 = f4_fma(g[fx], v[fx], h0); h1 = f4_fma(g[fx], v[fx + 1], h1); }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty_bar(s));
-        if (++s == NR) { s = 0; ph ^= 1u; }
-    };
     const int64_t par_stride = (int64_t)N * SH * SW * C;
     float4 h[5][2];
 #pragma unroll
-    for (int r = 0; r < 3; ++r) hrow(iy_first + r, h[r][0], h[r][1]);
+    for (int r = 0; r < 3; ++r) fir_hrow_down(ring, iy_first + r, vl, vm, vr, h[r]);
     for (int sy = SY0; sy < SY0 + rows_here; ++sy) {
         const int y0 = sy * 2;
-        hrow(y0 + 1, h[3][0], h[3][1]);
-        hrow(y0 + 2, h[4][0], h[4][1]);
-        if (active) {
-            const int64_t o = (((int64_t)n * SH + sy) * SW + sx) * C + c4 * 4;
-#pragma unroll
-            for (int a = 0; a < 2; ++a)
-#pragma unroll
-                for (int b = 0; b < 2; ++b) {
-                    float4 v = f4_scale(g[0], h[a][b]);
-#pragma unroll
-                    for (int r = 1; r < 4; ++r) v = f4_fma(g[r], h[a + r][b], v);
-                    if (y0 + a > H || x0 + b > W) v = z;        // beyond the (H+1)x(W+1) FIR output: zero pad
-                    uint2 hh, l;
-                    split_bf16x2(v.x, v.y, hh.x, l.x); split_bf16x2(v.z, v.w, hh.y, l.y);
-                    const int64_t off = (int64_t)(a * 2 + b) * par_stride + o;
-                    *reinterpret_cast<uint2*>(hi + off) = hh;
-                    *reinterpret_cast<uint2*>(lo + off) = l;
-                }
-        }
-#pragma unroll
-        for (int r = 0; r < 3; ++r) { h[r][0] = h[r + 2][0]; h[r][1] = h[r + 2][1]; }
+        fir_hrow_down(ring, y0 + 1, vl, vm, vr, h[3]);
+        fir_hrow_down(ring, y0 + 2, vl, vm, vr, h[4]);
+        const int64_t o = (((int64_t)n * SH + sy) * SW + sx) * C + c4 * 4;
+        fir_down_block(h, active, y0, x0, H, W, par_stride, hi + o, lo + o);
     }
 }
 
@@ -659,12 +601,12 @@ extern "C" int n3d_demod(const float* styles, const float* wsq, const int64_t* r
     return N3D_OK;
 }
 
-// Rows per thread strip of the FIR kernels: 16 (3 re-read halo rows per strip) for launches with >= 1024 threads per SM, halved
-// down to 4 for smaller ones.  Measured on B200 (tools/bench_layers.py): S=1 is 1.3-1.6x slower than S=4 at every size, S=64
-// loses on everything below 256^2.
-static int fir_strip_rows(int64_t threads_per_row, int rows) {
+// Rows per thread strip of the register-tiled FIR kernels: 16 (3 re-read halo rows per strip) for launches with >= 1024 threads per
+// SM, halved down to 4 for smaller ones.  Measured on B200 (tools/bench_layers.py): S=1 is 1.3-1.6x slower than S=4 at every size,
+// S=64 loses on everything below 256^2.
+static int fir_strip_rows(int64_t threads_per_row, int rows, int num_sms) {
     int S = 16;
-    while (S > 4 && threads_per_row * n3d_div_up(rows, S) < (int64_t)148 * 1024) S >>= 1;
+    while (S > 4 && threads_per_row * n3d_div_up(rows, S) < (int64_t)num_sms * 1024) S >>= 1;
     return min(S, rows);
 }
 
@@ -679,61 +621,99 @@ extern "C" int n3d_modulate_split(const float* x, int64_t npix_per_img, int N, i
     return N3D_OK;
 }
 
+// The streamed FIR kernels may run on this input: 16-byte aligned, and not switched off by N3D_FIR_STREAM=0 (register-tiled kernels
+// for every shape: A/B runs, and the reference the tests hold the streamed kernels to).  Read at every call, so that one process can
+// compare both forms.
+static bool fir_streamable(const float* x) {
+    const char* e = getenv("N3D_FIR_STREAM");
+    return (!e || atoi(e) != 0) && ((uintptr_t)x & 15) == 0;
+}
+
+// Kernel and geometry of one FIR launch.  rows > 0: the streamed kernel, tiles of `rows` x `cols` (output rows x columns up,
+// sub-pixel rows x columns down) through a ring of NR stages in `smem` bytes of dynamic shared memory.  rows == 0: the register-tiled
+// kernel in strips of S rows.
+struct FirPlan { int grid, rows, cols, NR, smem, S; };
+
+// FIR-up epilogue: streamed for the large layers -- (TC / 2) * (C / 4) == 256 consumer threads, at least one CTA per SM.
+static FirPlan fir_up_plan(const float* raw, int N, int H2, int W2, int C, int num_sms) {
+    FirPlan P{};
+    const int TC = (C >= 64 && C <= 512 && (2048 % C) == 0) ? 2048 / C : 0;
+    if (TC >= 4 && W2 % TC == 0 && fir_streamable(raw)) {
+        // rows per tile: the candidate with the best (fill of the last wave of 2 CTAs per SM) x (1 - vertical halo); measured sweep in
+        // DESIGN.md section 3.3.  The tiling does not change the arithmetic (results are bit-identical for every tile height).
+        double best = 0.0;
+        for (int tr = 32; tr <= 128; tr *= 2) {
+            if (H2 % tr) continue;
+            const int64_t ctas = (int64_t)N * (W2 / TC) * (H2 / tr);
+            if (ctas < num_sms) continue;
+            const double eff = (double)ctas / (double)(n3d_div_up(ctas, 2 * num_sms) * 2 * num_sms) * tr / (tr + 3);
+            if (eff > best) { best = eff; P.rows = tr; P.grid = (int)ctas; }
+        }
+    }
+    if (P.rows) {
+        const int row_bytes = (TC + 3) * C * 4;
+        P.cols = TC;
+        P.NR = min(4, (100 * 1024) / row_bytes);               // deeper rings measured 1-3 % slower (sweep 4 / 6 / 8 / 10)
+        P.smem = P.NR * row_bytes + 16 * P.NR;
+    } else {
+        P.S = fir_strip_rows((int64_t)N * (W2 / 2) * (C / 4), H2 / 2, num_sms);
+        P.grid = grid_for((int64_t)N * n3d_div_up(H2 / 2, P.S) * (W2 / 2) * (C / 4), 256, 16);
+    }
+    return P;
+}
+
+// FIR-down split: streamed for the large layers -- TSC * (C / 4) == 256 consumer threads, at least one CTA per SM.
+static FirPlan fir_down_plan(const float* x, int N, int H, int W, int C, int num_sms) {
+    FirPlan P{};
+    const int c4n = C / 4, SH = (H + 2) / 2, SW = (W + 2) / 2;
+    const int TSC = (c4n >= 8 && c4n <= 128 && 256 % c4n == 0) ? 256 / c4n : 0;
+    if (TSC && fir_streamable(x)) {
+        for (int ts = 32; ts >= 16; ts >>= 1) {
+            const int64_t ctas = (int64_t)N * n3d_div_up(SW, TSC) * n3d_div_up(SH, ts);
+            if (ctas >= num_sms) { P.rows = ts; P.grid = (int)ctas; break; }
+        }
+    }
+    if (P.rows) {
+        P.cols = TSC;
+        P.NR = 4;
+        P.smem = P.NR * (2 * TSC + 3) * C * 4 + 16 * P.NR;
+    } else {
+        P.S = fir_strip_rows((int64_t)N * SW * c4n, SH, num_sms);
+        P.grid = grid_for((int64_t)N * n3d_div_up(SH, P.S) * SW * c4n, 256, 16);
+    }
+    return P;
+}
+
+// EpiParams of one epilogue launch, after the checks the epilogue relies on: an lrelu / linear activation and float4-aligned outputs.
+// Errors name the entry point `who`.
+static int epi_params(EpiParams& E, const char* who, const float* dcoef, const float* bias, const float* noise, int64_t noise_nstride,
+                      float gain, float slope, float clamp, const N3DSplitOut out[2], float* out_f32, int f32_cstride, int f32_coff) {
+    N3D_CHECK_ARG(gain > 0.f && slope >= 0.f && slope <= 1.f, "%s: needs gain > 0 and 0 <= slope <= 1 (lrelu / linear)", who);
+    for (int k = 0; k < 2; ++k)
+        N3D_CHECK_ARG(!out[k].hi || (out[k].cstride % 4 == 0 && out[k].coff % 4 == 0), "%s: unaligned split output", who);
+    N3D_CHECK_ARG(!out_f32 || (f32_cstride % 4 == 0 && f32_coff % 4 == 0), "%s: unaligned fp32 output", who);
+    E = EpiParams{dcoef, bias, noise, noise_nstride, gain, slope, clamp, {out[0], out[1]}, out_f32, f32_cstride, f32_coff};
+    return N3D_OK;
+}
+
 extern "C" int n3d_fir_up_epilogue(const float* raw, int N, int H2, int W2, int C, const float* dcoef, const float* bias,
                                    const float* noise, int64_t noise_nstride, float gain, float slope, float clamp,
                                    const N3DSplitOut out[2], float* out_f32, int f32_cstride, int f32_coff, void* stream) {
     N3D_CHECK_ARG(raw && out, "n3d_fir_up_epilogue: null pointer");
     N3D_CHECK_ARG(C % 4 == 0, "n3d_fir_up_epilogue: C must be a multiple of 4");
-    N3D_CHECK_ARG(gain > 0.f && slope >= 0.f && slope <= 1.f, "n3d_fir_up_epilogue: needs gain > 0 and 0 <= slope <= 1 (lrelu / linear)");
     EpiParams E;
-    E.dcoef = dcoef; E.bias = bias; E.noise = noise; E.noise_nstride = noise_nstride; E.gain = gain; E.slope = slope; E.clamp = clamp;
-    E.out[0] = out[0]; E.out[1] = out[1]; E.out_f32 = out_f32; E.f32_cstride = f32_cstride; E.f32_coff = f32_coff;
-    for (int k = 0; k < 2; ++k)
-        N3D_CHECK_ARG(!E.out[k].hi || ((E.out[k].cstride % 4 == 0) && (E.out[k].coff % 4 == 0)), "n3d_fir_up_epilogue: unaligned split output");
-    N3D_CHECK_ARG(!out_f32 || (f32_cstride % 4 == 0 && f32_coff % 4 == 0), "n3d_fir_up_epilogue: unaligned fp32 output");
+    if (int e = epi_params(E, "n3d_fir_up_epilogue", dcoef, bias, noise, noise_nstride, gain, slope, clamp, out, out_f32, f32_cstride, f32_coff))
+        return e;
     N3D_CHECK_ARG(H2 % 2 == 0 && W2 % 2 == 0, "n3d_fir_up_epilogue: output size must be even");
-    {   // streamed variant (fir_up_stream_kernel) for the large layers: (TC / 2) * (C / 4) == 256 consumer threads, >= one CTA per SM
-        const char* e = getenv("N3D_FIR_STREAM");               // N3D_FIR_STREAM=0: the register-tiled kernel (A/B diagnostics, tests)
-        const int stream_mode = e ? atoi(e) : 1;
-        const int TC = (C >= 64 && C <= 512 && (2048 % C) == 0) ? 2048 / C : 0;
-        // rows per tile: the candidate with the best (fill of the last wave of 2 CTAs per SM) x (1 - vertical halo); measured sweep in
-        // DESIGN.md section 3.3.  The tiling does not change the arithmetic (results are bit-identical for every TR).
-        int TR = 0;
-        if (TC >= 4 && W2 % TC == 0) {
-            double best = 0.0;
-            for (int tr = 32; tr <= 128; tr *= 2) {
-                if (H2 % tr) continue;
-                const int64_t ctas = (int64_t)N * (W2 / TC) * (H2 / tr);
-                if (ctas < 148) continue;
-                const double eff = (double)ctas / (double)(n3d_div_up(ctas, 296) * 296) * tr / (tr + 3);
-                if (eff > best) { best = eff; TR = tr; }
-            }
-        }
-        if (const char* t = getenv("N3D_FIR_TR")) { TR = atoi(t); if (TR > H2) TR = H2; }      // tuning sweep only
-        if (stream_mode && TR > 0 && TC >= 4 && W2 % TC == 0 && H2 % TR == 0 && ((uintptr_t)raw & 15) == 0 &&
-            (int64_t)N * (W2 / TC) * (H2 / TR) >= 148) {
-            const int row_bytes = (TC + 3) * C * 4;
-            int NR = min(4, (100 * 1024) / row_bytes);         // deeper rings measured 1-3 % slower (sweep 4 / 6 / 8 / 10)
-            if (const char* t = getenv("N3D_FIR_NR")) NR = max(3, min(atoi(t), (110 * 1024) / row_bytes));
-            const int smem = NR * row_bytes + 16 * NR;
-            N3DDeviceState* D = n3d_device_state();
-            if (!D) return N3D_ERR_CUDA;
-            if (!(D->configured & N3D_CFG_FIR_STREAM)) {
-                if (cudaFuncSetAttribute(fir_up_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024) != cudaSuccess) {
-                    n3d_set_error("n3d_fir_up_epilogue: cannot raise dynamic shared memory to 112 KiB");
-                    return N3D_ERR_CUDA;
-                }
-                D->configured |= N3D_CFG_FIR_STREAM;
-            }
-            fir_up_stream_kernel<<<N * (W2 / TC) * (H2 / TR), kFsThreads, smem, (cudaStream_t)stream>>>(raw, N, H2, W2, C, TC, TR, NR, E);
-            N3D_CHECK_LAUNCH("n3d_fir_up_epilogue");
-            return N3D_OK;
-        }
+    N3DDeviceState* D = n3d_device_state();
+    if (!D) return N3D_ERR_CUDA;
+    const FirPlan P = fir_up_plan(raw, N, H2, W2, C, D->num_sms);
+    if (P.rows) {
+        if (int e = n3d_smem_optin(D, N3D_CFG_FIR_STREAM, (const void*)fir_up_stream_kernel, kFsSmemLimit, "n3d_fir_up_epilogue")) return e;
+        fir_up_stream_kernel<<<P.grid, kFsThreads, P.smem, (cudaStream_t)stream>>>(raw, N, H2, W2, C, P.cols, P.rows, P.NR, E);
+    } else {
+        fir_up_epilogue_kernel<<<P.grid, 256, 0, (cudaStream_t)stream>>>(raw, N, H2, W2, C, P.S, E);
     }
-    const int S = fir_strip_rows((int64_t)N * (W2 / 2) * (C / 4), H2 / 2);
-    const int64_t total = (int64_t)N * n3d_div_up(H2 / 2, S) * (W2 / 2) * (C / 4);
-    // 2 output columns per thread: measured best on B200 (1 column: +23 % time despite 1.5x the occupancy, 4 columns: +15 %)
-    fir_up_epilogue_kernel<2><<<grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream>>>(raw, N, H2, W2, C, S, E);
     N3D_CHECK_LAUNCH("n3d_fir_up_epilogue");
     return N3D_OK;
 }
@@ -743,13 +723,9 @@ extern "C" int n3d_splitk_epilogue(const float* partial, int S, int64_t split_st
                                    const N3DSplitOut out[2], float* out_f32, int f32_cstride, int f32_coff, void* stream) {
     N3D_CHECK_ARG(partial && out && S >= 1 && N > 0 && H > 0 && W > 0, "n3d_splitk_epilogue: bad args");
     N3D_CHECK_ARG(C % 4 == 0 && split_stride % 4 == 0 && ((uintptr_t)partial & 15) == 0, "n3d_splitk_epilogue: C and the split stride must be multiples of 4");
-    N3D_CHECK_ARG(gain > 0.f && slope >= 0.f && slope <= 1.f, "n3d_splitk_epilogue: needs gain > 0 and 0 <= slope <= 1 (lrelu / linear)");
     EpiParams E;
-    E.dcoef = dcoef; E.bias = bias; E.noise = noise; E.noise_nstride = noise_nstride; E.gain = gain; E.slope = slope; E.clamp = clamp;
-    E.out[0] = out[0]; E.out[1] = out[1]; E.out_f32 = out_f32; E.f32_cstride = f32_cstride; E.f32_coff = f32_coff;
-    for (int k = 0; k < 2; ++k)
-        N3D_CHECK_ARG(!E.out[k].hi || ((E.out[k].cstride % 4 == 0) && (E.out[k].coff % 4 == 0)), "n3d_splitk_epilogue: unaligned split output");
-    N3D_CHECK_ARG(!out_f32 || (f32_cstride % 4 == 0 && f32_coff % 4 == 0), "n3d_splitk_epilogue: unaligned fp32 output");
+    if (int e = epi_params(E, "n3d_splitk_epilogue", dcoef, bias, noise, noise_nstride, gain, slope, clamp, out, out_f32, f32_cstride, f32_coff))
+        return e;
     const int64_t total = (int64_t)N * H * W * (C / 4);
     splitk_epilogue_kernel<<<grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream>>>(partial, S, split_stride, N, H, W, C, E);
     N3D_CHECK_LAUNCH("n3d_splitk_epilogue");
@@ -759,34 +735,16 @@ extern "C" int n3d_splitk_epilogue(const float* partial, int S, int64_t split_st
 extern "C" int n3d_fir_down_split(const float* x, int N, int H, int W, int C, void* hi, void* lo, void* stream) {
     N3D_CHECK_ARG(x && hi && lo, "n3d_fir_down_split: null pointer");
     N3D_CHECK_ARG(C % 4 == 0 && H % 2 == 0 && W % 2 == 0, "n3d_fir_down_split: C %% 4 and even H, W required");
-    {   // streamed variant for the large layers (see fir_down_stream_kernel); N3D_FIR_STREAM=0: the register-tiled kernel
-        const char* e = getenv("N3D_FIR_STREAM");
-        const int c4n = C / 4, SH = (H + 2) / 2, SW = (W + 2) / 2;
-        const int TSC = (c4n >= 8 && c4n <= 128 && 256 % c4n == 0) ? 256 / c4n : 0;
-        int TS = 0;
-        for (int ts = 32; ts >= 16 && TSC; ts >>= 1)
-            if ((int64_t)N * n3d_div_up(SW, TSC) * n3d_div_up(SH, ts) >= 148) { TS = ts; break; }
-        if ((!e || atoi(e) != 0) && TS > 0 && ((uintptr_t)x & 15) == 0) {
-            const int row_bytes = (2 * TSC + 3) * C * 4, NR = 4;
-            const int smem = NR * row_bytes + 16 * NR;
-            N3DDeviceState* D = n3d_device_state();
-            if (!D) return N3D_ERR_CUDA;
-            if (!(D->configured & N3D_CFG_FIR_DOWN_STREAM)) {
-                if (cudaFuncSetAttribute(fir_down_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024) != cudaSuccess) {
-                    n3d_set_error("n3d_fir_down_split: cannot raise dynamic shared memory to 112 KiB");
-                    return N3D_ERR_CUDA;
-                }
-                D->configured |= N3D_CFG_FIR_DOWN_STREAM;
-            }
-            fir_down_stream_kernel<<<N * n3d_div_up(SW, TSC) * n3d_div_up(SH, TS), kFsThreads, smem, (cudaStream_t)stream>>>(
-                x, N, H, W, C, TSC, TS, NR, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo);
-            N3D_CHECK_LAUNCH("n3d_fir_down_split");
-            return N3D_OK;
-        }
+    N3DDeviceState* D = n3d_device_state();
+    if (!D) return N3D_ERR_CUDA;
+    const FirPlan P = fir_down_plan(x, N, H, W, C, D->num_sms);
+    if (P.rows) {
+        if (int e = n3d_smem_optin(D, N3D_CFG_FIR_DOWN_STREAM, (const void*)fir_down_stream_kernel, kFsSmemLimit, "n3d_fir_down_split")) return e;
+        fir_down_stream_kernel<<<P.grid, kFsThreads, P.smem, (cudaStream_t)stream>>>(x, N, H, W, C, P.cols, P.rows, P.NR, (__nv_bfloat16*)hi,
+                                                                                      (__nv_bfloat16*)lo);
+    } else {
+        fir_down_split_kernel<<<P.grid, 256, 0, (cudaStream_t)stream>>>(x, N, H, W, C, P.S, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo);
     }
-    const int S = fir_strip_rows((int64_t)N * ((W + 2) / 2) * (C / 4), (H + 2) / 2);
-    const int64_t total = (int64_t)N * n3d_div_up((H + 2) / 2, S) * ((W + 2) / 2) * (C / 4);
-    fir_down_split_kernel<<<grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream>>>(x, N, H, W, C, S, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo);
     N3D_CHECK_LAUNCH("n3d_fir_down_split");
     return N3D_OK;
 }

@@ -537,13 +537,7 @@ extern "C" int n3d_fill_mouth(float* alpha, int NI, int H, int W, void* stream) 
     N3D_CHECK_ARG((int64_t)H * (W + 4) <= 200 * 1024, "n3d_fill_mouth: image %dx%d too large for the shared-memory state map", H, W);
     N3DDeviceState* D = n3d_device_state();
     if (!D) return N3D_ERR_CUDA;
-    if (!(D->configured & N3D_CFG_FILL_MOUTH)) {
-        if (cudaFuncSetAttribute(fill_mouth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
-            n3d_set_error("n3d_fill_mouth: cannot raise dynamic shared memory");
-            return N3D_ERR_CUDA;
-        }
-        D->configured |= N3D_CFG_FILL_MOUTH;
-    }
+    if (int e = n3d_smem_optin(D, N3D_CFG_FILL_MOUTH, (const void*)fill_mouth_kernel, 200 * 1024, "n3d_fill_mouth")) return e;
     fill_mouth_kernel<<<NI, 1024, (size_t)H * (W + 4), (cudaStream_t)stream>>>(alpha, H, W);
     N3D_CHECK_LAUNCH("n3d_fill_mouth");
     return N3D_OK;

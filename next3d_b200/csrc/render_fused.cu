@@ -1244,10 +1244,7 @@ int n3d_render_floor_launch(const N3DRender* p, int kind, float* sink, void* str
     const int grid = (int)(K.total_groups < D->num_sms ? K.total_groups : D->num_sms);
     if (kind == 0) {
         const size_t smem = 32768 + kWarps * kTapBytesPerWarp + 1024;
-        if (cudaFuncSetAttribute(gather_floor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-            n3d_set_error("n3d_render_floor: cannot raise dynamic shared memory");
-            return N3D_ERR_CUDA;
-        }
+        if (int e = n3d_smem_optin(D, N3D_CFG_FLOOR_GATHER, (const void*)gather_floor_kernel, (int)smem, "n3d_render_floor")) return e;
         gather_floor_kernel<<<grid, kThreads, smem, (cudaStream_t)stream>>>(K, sink);
     } else {
         const long long samples = (long long)p->N * K.M * (p->depth_coarse + p->depth_fine);
@@ -1278,16 +1275,9 @@ int n3d_render_fused_launch(const N3DRender* p, void* stream, int mode) {
     N3DDeviceState* D = n3d_device_state();
     if (!D) return N3D_ERR_CUDA;
     const size_t smem = (size_t)kSmemBytes + 1024;
-    const unsigned bit = L == 16 ? N3D_CFG_RENDER16 : N3D_CFG_RENDER32;
-    if (!(D->configured & bit)) {
-        const cudaError_t e = L == 16 ? cudaFuncSetAttribute(render_fused_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                                      : cudaFuncSetAttribute(render_fused_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) {
-            n3d_set_error("n3d_render_rays: cannot raise dynamic shared memory: %s", cudaGetErrorString(e));
-            return N3D_ERR_CUDA;
-        }
-        D->configured |= bit;
-    }
+    if (int e = L == 16 ? n3d_smem_optin(D, N3D_CFG_RENDER16, (const void*)render_fused_kernel<16>, (int)smem, "n3d_render_rays")
+                        : n3d_smem_optin(D, N3D_CFG_RENDER32, (const void*)render_fused_kernel<32>, (int)smem, "n3d_render_rays"))
+        return e;
     const int grid = (int)(K.total_groups < D->num_sms ? K.total_groups : D->num_sms);
     if (L == 16) render_fused_kernel<16><<<grid, kThreads, smem, (cudaStream_t)stream>>>(K);
     else render_fused_kernel<32><<<grid, kThreads, smem, (cudaStream_t)stream>>>(K);
@@ -1314,14 +1304,9 @@ int n3d_points_fused_launch(const float* planes, int N, int PH, int PW, const fl
     N3DDeviceState* D = n3d_device_state();
     if (!D) return N3D_ERR_CUDA;
     const size_t smem = (size_t)kSmemBytes + 1024;
-    if (!(D->configured & N3D_CFG_POINTS)) {
-        if (cudaFuncSetAttribute(points_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-            cudaFuncSetAttribute(points_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-            n3d_set_error("n3d_sample_points: cannot raise dynamic shared memory");
-            return N3D_ERR_CUDA;
-        }
-        D->configured |= N3D_CFG_POINTS;
-    }
+    if (int e = rgb ? n3d_smem_optin(D, N3D_CFG_POINTS_RGB, (const void*)points_fused_kernel<true>, (int)smem, "n3d_sample_points")
+                    : n3d_smem_optin(D, N3D_CFG_POINTS, (const void*)points_fused_kernel<false>, (int)smem, "n3d_sample_points"))
+        return e;
     const long long tiles = (K.total + 127) / 128;
     const int grid = (int)(tiles < D->num_sms ? tiles : D->num_sms);
     if (rgb) points_fused_kernel<true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(K);

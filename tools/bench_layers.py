@@ -51,13 +51,6 @@ def main(tag):
             os.environ['N3D_FIR_STREAM'] = mode
             us = timeit(lambda: K.fir_up_epilogue(raw, cout, d, b, nz, 2 ** 0.5, 0.2, 256.0, outs=outs))
             print(f'fir_up  C={cout:4d} out {2 * res:3d}^2 stream={mode} {us:8.1f} us  {gb / us * 1e-3:6.0f} GB/s')
-        if os.environ.get('FIR_SWEEP'):
-            for tr in (16, 32, 64, 128):
-                for nr in (4, 6, 8, 10):
-                    os.environ['N3D_FIR_TR'], os.environ['N3D_FIR_NR'] = str(tr), str(nr)
-                    us = timeit(lambda: K.fir_up_epilogue(raw, cout, d, b, nz, 2 ** 0.5, 0.2, 256.0, outs=outs))
-                    print(f'   TR={tr:3d} NR={nr:2d} {us:8.1f} us  {gb / us * 1e-3:6.0f} GB/s')
-            os.environ.pop('N3D_FIR_TR'); os.environ.pop('N3D_FIR_NR')
         os.environ.pop('N3D_FIR_STREAM')
     if os.environ.get('FIR_ONLY'):
         return
